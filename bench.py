@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — LM iterations/s of the LiDAR-visual BA hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C] [--dump-outputs DIR]
 
 A *step* — the same for both arms, written into `config.step` of both lines — is ONE full LM iteration of the whole hot path on
 one synthetic problem, started from the initial state (SURVEY.md §8d):
@@ -115,14 +115,27 @@ def algorithmic_bytes(p, lid_counts, vis_counts, n_active):
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm
+def step_outputs(poses, a, q, t, X, b):
+    """what one step hands its caller, under the names --dump-outputs writes; a, b: the two paths' summaries"""
+    return {"lidar_poses": poses, "lidar_cost": np.array([a["cost_first"], a["cost_last"]]),
+            "visual_q": q, "visual_t": t, "visual_X": X, "visual_cost": np.array([b["cost_first"], b["cost_last"]])}
+
+
+def dump_outputs(out_dir, outputs):
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a, np.float64))
+
+
 def cpu_pass(p, threads_a, threads_b):
-    """one full LM pass of each path on the full problem with the CPU restatement; ms per pass (A, B)"""
+    """one full LM pass of each path on the full problem with the CPU restatement; ms per pass (A, B) and step_outputs"""
     from oracle import cpu_ref
-    _, a = cpu_ref.lidar_lm(p["vox_ptr"], p["pose_idx"], p["clusters"], p["poses"], max_iter=1, rel_tol=-1.0, threads=threads_a)
-    _, _, _, b = cpu_ref.visual_lm(*[p[k] for k in VKEYS], max_iter=1, threads=threads_b, function_tolerance=-1.0)
+    poses, a = cpu_ref.lidar_lm(p["vox_ptr"], p["pose_idx"], p["clusters"], p["poses"], max_iter=1, rel_tol=-1.0, threads=threads_a)
+    q, t, X, b = cpu_ref.visual_lm(*[p[k] for k in VKEYS], max_iter=1, threads=threads_b, function_tolerance=-1.0)
     tA = a["ms_build"] + a["ms_solve"] + a["ms_residual"]
     tB = b["ms_build"] + b["ms_solve"] + b["ms_residual"]
-    return tA, tB
+    return tA, tB, step_outputs(poses, a, q, t, X, b)
 
 
 def cpu_thread_sweep(p):
@@ -132,7 +145,7 @@ def cpu_thread_sweep(p):
     cand = sorted({t for t in (8, 16, 32, 64, hw) if t <= max(hw, 16)})
     sweep = {}
     for t in cand:
-        tA, tB = cpu_pass(p, t, t)
+        tA, tB, _ = cpu_pass(p, t, t)
         sweep[str(t)] = {"ms_A": round(tA, 1), "ms_B": round(tB, 1)}
     best_a = min(cand, key=lambda t: sweep[str(t)]["ms_A"])
     best_b = min(cand, key=lambda t: sweep[str(t)]["ms_B"])
@@ -144,9 +157,11 @@ def run_reference(args, p, cfg):
     ta, tb, sweep, hw = cpu_thread_sweep(p)
     times = []
     for i in range(args.warmup + args.steps):
-        tA, tB = cpu_pass(p, ta, tb)
+        tA, tB, outputs = cpu_pass(p, ta, tb)
         if i >= args.warmup:
             times.append((tA + tB) / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     mean = sum(times) / len(times)
     val = 1.0 / mean
     # e2e of this arm: the same call of each boundary to the reference's caps, time / passes (host memory only: no copies)
@@ -212,6 +227,8 @@ def measure_resident(pkg, torch, p, device, steps, warmup, barrier, rank):
     barrier()
     wall = time.perf_counter() - wall0
     nccl_bytes = pkg.comm_bytes_sent() / steps
+    q, t, X = Vz.get_state()                                     # what the last timed step left, before the full LM below moves it
+    outputs = step_outputs(L.get_poses(), sa, q, t, X, sb)
     ra, rb = L.owned_rows(), Vz.owned_rows()
     # full LM to the reference's caps (BASELINE configs[2]), device resident
     L.reset_lm(None); L.reset_state(); fa2 = L.iterate(2)        # the LM amplifies rounding differences from iteration to iteration
@@ -220,7 +237,7 @@ def measure_resident(pkg, torch, p, device, steps, warmup, barrier, rank):
     out = {"cost_A_after_2": fa2["cost_last"],"host_s": host_s, "wall": wall, "launches": launches, "dev_ms": {k: v / steps for k, v in dev_ms.items()},
            "full_A": fa, "full_B": fb, "lid_counts": L.counts(nonzero=True), "vis_counts": Vz.counts(),
            "n_active": len(Vz.structure()[0]), "structA": L.structure(), "structB": Vz.structure(),
-           "nccl_bytes_per_step": nccl_bytes, "owned_rows_A": ra, "owned_rows_B": rb}
+           "nccl_bytes_per_step": nccl_bytes, "owned_rows_A": ra, "owned_rows_B": rb, "outputs": outputs}
     L.close(); Vz.close()
     del flush
     return out
@@ -242,7 +259,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the GPU-vs-CPU full-LM parity check at the benchmarked config")
     ap.add_argument("--no-voxel-map", action="store_true", help="skip the boundary-B3 (voxel map) side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (poses, cameras, points, costs) as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -343,6 +364,8 @@ def main():
                      "note": "lvba_lidar_lm(max_iter=1) + lvba_visual_lm(max_iter=1): set-up and upload of the whole problem for ONE pass"}
 
     rc = 0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, R["outputs"])
     if rank == 0:
         ab = algorithmic_bytes(p, R["lid_counts"], R["vis_counts"], R["n_active"])
         try:
@@ -432,7 +455,7 @@ def main():
                 rc = 3
         if world == 1 and not args.no_cpu_baseline:
             ta_, tb_, sweep, hw = cpu_thread_sweep(p)
-            tA, tB = cpu_pass(p, ta_, tb_)
+            tA, tB, _ = cpu_pass(p, ta_, tb_)
             line["cpu_baseline"] = {"value": 1e3 / (tA + tB), "unit": UNIT, "cores": max(ta_, tb_), "threads_path_A": ta_, "threads_path_B": tb_,
                                     "host_hardware_threads": hw, "kind": "port", "thread_sweep_ms_per_pass": sweep,
                                     "sample": "1 full LM pass of path A + 1 of path B on the full problem (oracle/cpu_ref.cpp) at the fastest thread "

@@ -18,7 +18,7 @@ ROOT = Path(__file__).resolve().parents[1]
 def test_two_rank_sharded_run_matches_the_oracle():
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     port = 29600 + os.getpid() % 1000
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", str(port), str(ROOT / "tools" / "mgpu_check.py"), "B"]

@@ -9,8 +9,9 @@ is the reference's).  Here, without a GPU:
   1. the numpy oracles (oracle/*.py) reproduce the file            -> the restatements equal the source they restate
   2. the C++ port oracle/cpu_ref.cpp (the bench's CPU arm) does too  -> the timed CPU arm computes what the reference does
   3. the device passes, run through the host policy (tests/emu/), do too (voxel map, anchor clouds, >128-pose voxel pass)
-  4. where oracle/_ref/libbalm_ref.so can be built (this container), the file is regenerated and must come out bit for bit,
-     and further seeded problems are compared live (reference source vs oracle) at sizes the fixture does not hold.
+  4. further seeded problems, at sizes the fixture does not hold, against what the reference source computed from them
+     (tests/golden/ref_live_balm.npz, written by tests/golden/make_golden_ref_live.py); where oracle/_ref/libbalm_ref.so is
+     built, the fixture is also regenerated and must come out bit for bit.
 
 The CUDA path is held against the same file in tests/test_zzz_ref_gpu.py.  Tolerances: integer / key / count data exact;
 float64 sums whose order differs 1e-12 relative; quantities behind the eigen-decomposition of P/N - v v^T (lambda_0, g, H:
@@ -30,8 +31,15 @@ from oracle import anchor_oracle as ao, balm_ref, depth_oracle as dep, lidar_ora
 import test_anchor_emu, test_big_voxel_emu, test_voxel_emu  # noqa: E402,E401
 
 G = np.load(ROOT / "tests" / "golden" / "ref_balm.npz")
+LIVE = ROOT / "tests" / "golden" / "ref_live_balm.npz"
 
-needs_ref = pytest.mark.skipif(not balm_ref.available(), reason="oracle/_ref/libbalm_ref.so needs /root/reference (not on the GPU box)")
+needs_ref = pytest.mark.skipif(not balm_ref.available(), reason="oracle/_ref/libbalm_ref.so is built only where the original sources are readable")
+
+
+def recorded(tag):
+    """What the ref_* function below returned for case `tag` when the fixture was written."""
+    with np.load(LIVE) as f:
+        return {k[len(tag) + 2:]: f[k] for k in f.files if k.startswith(tag + "__")}
 
 
 def csr(tag):
@@ -313,31 +321,91 @@ def test_fixture_is_what_the_reference_source_computes_bit_for_bit():
     assert exact or os.environ.get("LVBA_ALLOW_OTHER_HOST", "1") == "1"     # on the machine that wrote the file the regeneration is bit for bit
 
 
-@needs_ref
-@pytest.mark.parametrize("W,V,seed", [(6, 40, 1), (50, 1500, 2), (120, 3000, 3)])
-def test_live_hessian_and_lm_reference_source_vs_numpy(W, V, seed):
+# The ref_* functions run the reference source on one case; tests/golden/make_golden_ref_live.py stores what they return.
+HESSIAN_CASES = [(6, 40, 1), (50, 1500, 2), (120, 3000, 3)]
+VOXEL_MAP_CASES = [(31, 1.0), (32, 0.5), (33, 2.0)]
+H_FULL_MAX_W = 6         # a larger H is stored as H Z, its diagonal blocks and 200 of the others: the whole of it would not fit the file.
+#                          The stored blocks are checked entry by entry at the tolerance; an entry outside them only through H Z, which
+#                          misses an error in a single entry below about sum|Z[:, j]| / |Z[i, j]| (some 6W) times the tolerance.
+
+
+def hessian_problem(W, V, seed):
     p = synth.make_problem(W, V, 0, seed=seed, visual=False)
-    a = (p["vox_ptr"], p["pose_idx"], p["clusters"], p["poses"])
+    return p["vox_ptr"], p["pose_idx"], p["clusters"], p["poses"]
+
+
+def hessian_probe(W, seed):
+    """The fixed test matrix Z and the (i, j), i > j, of the off-diagonal blocks kept of a Hessian too large to store whole."""
+    rng = np.random.default_rng(1000 + seed)
+    Z = rng.standard_normal((6 * W, 8))
+    lower = np.array([(i, j) for i in range(W) for j in range(i)])
+    return Z, lower[np.sort(rng.choice(len(lower), size=min(len(lower), 200), replace=False))]
+
+
+def blocks_at(H, ij):
+    return np.array([H[6 * i:6 * i + 6, 6 * j:6 * j + 6] for i, j in ij])
+
+
+def ref_hessian(W, V, seed):
+    a = hessian_problem(W, V, seed)
     res, g, H, kept = balm_ref.lidar_hessian(*a, threads=(seed % 2 == 0))
+    out = dict(res=res, g=g, kept=kept, lm_poses=balm_ref.lidar_damping_iter(*a))
+    if W <= H_FULL_MAX_W:
+        out["H"] = H
+    else:
+        Z, pick = hessian_probe(W, seed)
+        out.update(HZ=H @ Z, H_absmax=np.abs(H).max(), H_diag=blocks_at(H, [(i, i) for i in range(W)]), H_pick=blocks_at(H, pick))
+    return out
+
+
+@pytest.mark.parametrize("W,V,seed", HESSIAN_CASES)
+def test_live_hessian_and_lm_reference_source_vs_numpy(W, V, seed):
+    a = hessian_problem(W, V, seed)
+    R = recorded(f"hessian_{seed}")
+    res, g, kept = float(R["res"]), R["g"], int(R["kept"])
     r, g_o, blocks = lo.acc_evaluate2(*a, W)
     H_o = lo.assemble_dense(blocks, W)
     res_sum = res * kept if seed % 2 == 0 else res
+    tol = 1e-9 * np.abs(H_o).max()
     assert kept == V and abs(res_sum - r) <= 1e-9 * abs(r)
-    assert np.abs(g - g_o).max() <= 1e-9 * np.abs(g_o).max() and np.abs(H - H_o).max() <= 1e-9 * np.abs(H_o).max()
+    assert np.abs(g - g_o).max() <= 1e-9 * np.abs(g_o).max()
+    if "H" in R:
+        assert np.abs(R["H"] - H_o).max() <= tol
+    else:
+        Z, pick = hessian_probe(W, seed)
+        assert abs(float(R["H_absmax"]) - np.abs(H_o).max()) <= tol
+        assert np.all(np.abs(R["HZ"] - H_o @ Z) <= tol * np.abs(Z).sum(0))      # implied by every entry within tol, not the converse
+        assert np.abs(R["H_diag"] - blocks_at(H_o, [(i, i) for i in range(W)])).max() <= tol
+        assert np.abs(R["H_pick"] - blocks_at(H_o, pick)).max() <= tol
     poses, _ = lo.damping_iter(*a)
-    assert np.abs(balm_ref.lidar_damping_iter(*a) - poses).max() <= 1e-9
+    assert np.abs(R["lm_poses"] - poses).max() <= 1e-9
 
 
-@needs_ref
-@pytest.mark.parametrize("seed,voxel_size", [(31, 1.0), (32, 0.5), (33, 2.0)])
-def test_live_voxel_map_reference_source_vs_numpy(seed, voxel_size):
-    scans, poses = synth.make_scan_scene(seed, W=6, n_per_scan=2000)
+def scan_scene(seed):
+    return synth.make_scan_scene(seed, W=6, n_per_scan=2000)
+
+
+def ref_voxel_map(seed, voxel_size):
+    scans, poses = scan_scene(seed)
     m = balm_ref.Map(scans, poses, voxel_size)
     vp, pi, cl, meta = m.export()
+    m.close()
+    path = np.full((len(meta["path"]), max([1] + [len(p) for p in meta["path"]])), -1, np.int64)
+    for k, p in enumerate(meta["path"]):
+        path[k, :len(p)] = p
+    rel = ao.rel_poses(poses, np.array([0, len(scans)]))
+    return dict(vox_ptr=vp, pose_idx=pi, clusters=cl, key=meta["key"], layer=meta["layer"], path=path,
+                anchor_cloud_sorted=lex(balm_ref.anchor_cloud(scans, rel, 0.2)))
+
+
+@pytest.mark.parametrize("seed,voxel_size", VOXEL_MAP_CASES)
+def test_live_voxel_map_reference_source_vs_numpy(seed, voxel_size):
+    scans, poses = scan_scene(seed)
+    R = recorded(f"voxel_map_{seed}")
     ovp, opi, ocl, ometa = vox.voxelize_literal(scans, poses, voxel_size)
-    assert np.array_equal(vp, ovp) and np.array_equal(pi, opi) and np.abs(cl - ocl).max() <= 1e-12 * np.abs(ocl).max()
-    assert np.array_equal(meta["key"], ometa["key"]) and meta["path"] == list(ometa["path"]) and np.array_equal(meta["layer"], ometa["layer"])
+    assert np.array_equal(R["vox_ptr"], ovp) and np.array_equal(R["pose_idx"], opi) and np.abs(R["clusters"] - ocl).max() <= 1e-12 * np.abs(ocl).max()
+    path = [tuple(int(x) for x in p if x >= 0) for p in R["path"]]
+    assert np.array_equal(R["key"], ometa["key"]) and path == [tuple(p) for p in ometa["path"]] and np.array_equal(R["layer"], ometa["layer"])
     win_ptr = np.array([0, len(scans)])
     rel = ao.rel_poses(poses, win_ptr)
-    assert np.array_equal(lex(balm_ref.anchor_cloud(scans, rel, 0.2)), lex(ao.anchor_clouds_literal(scans, rel, win_ptr, 0.2)[0]))
-    m.close()
+    assert np.array_equal(R["anchor_cloud_sorted"], lex(ao.anchor_clouds_literal(scans, rel, win_ptr, 0.2)[0]))

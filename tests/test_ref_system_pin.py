@@ -18,7 +18,10 @@ stand-in library headers of oracle/ref_shim/ (own code; what that leaves open: r
      sigma 0.5 px / 0.01 m, 50 iterations DENSE_SCHUR, default tolerances; the points that enter are exactly the usable tracks with a
      valid plane, their planes those of the voxel oracle on the oracle's anchor clouds (live test: the scene is rebuilt, not stored)
 
-Where oracle/_ref/liblvba_system_ref.so can be built (this container) the file is regenerated and must come out bit for bit.
+The tests named *_live_* / *differential* / *reference_reader* / *reference_loader* / *real_container* / *reference_writer* compare with
+what the reference source computed from their inputs, stored in tests/golden/ref_live_system.npz by tests/golden/make_golden_ref_live.py
+(the ref_* functions below make those calls).  Where oracle/_ref/liblvba_system_ref.so is built, ref_system.npz is also regenerated and
+must come out bit for bit.
 """
 import os
 import sys
@@ -35,7 +38,19 @@ from oracle import anchor_oracle as ao, depth_oracle as dep, fuse_oracle as fo, 
 import test_depth_emu  # noqa: E402
 
 G = np.load(ROOT / "tests" / "golden" / "ref_system.npz")
-needs_ref = pytest.mark.skipif(not sr.available(), reason="oracle/_ref/liblvba_system_ref.so needs /root/reference (not on the GPU box)")
+LIVE = ROOT / "tests" / "golden" / "ref_live_system.npz"
+needs_ref = pytest.mark.skipif(not sr.available(), reason="oracle/_ref/liblvba_system_ref.so is built only where the original sources are readable")
+
+
+def recorded(tag):
+    """What the ref_* function of case `tag` returned when the fixture was written."""
+    with np.load(LIVE) as f:
+        return {k[len(tag) + 2:]: f[k] for k in f.files if k.startswith(tag + "__")}
+
+
+def flat(arrays):
+    """A list of arrays as (concatenation, CSR pointer)."""
+    return np.concatenate(arrays), np.r_[0, np.cumsum([len(a) for a in arrays])]
 
 
 def split(flat, ptr):
@@ -124,25 +139,40 @@ def test_lidar_half_equals_reference_source(use_rel):
         assert np.abs(G["L_final_poses_rel"] - G["L_final_poses"]).max() > 1e-5       # the switch does something
 
 
-@needs_ref
-@pytest.mark.parametrize("seed,W,win,use_rel,stage1,index", [(31, 10, 4, False, True, [0, 0, 0, 0, 1, 1, 1, 1, 2, 2]), (32, 10, 4, True, True, [0, 0, 0, 0, 1, 1, 1, 1, 2, 2]),
-                                                             (33, 7, 3, True, False, [0, 0, 0, 1, 1, 1, -1])])
-def test_lidar_half_live_ragged_windows_and_stage_switches(seed, W, win, use_rel, stage1, index):
-    """A last window shorter than the others, a last window of ONE frame (no voxel can see two poses: skipped, its frame keeps the odometry pose),
-    BALM_stage1/enable = false, both settings of use_window_ba_rel: the reference's runLidarBA, run live, against the oracle chain."""
+RAGGED_CASES = [(31, 10, 4, False, True, [0, 0, 0, 0, 1, 1, 1, 1, 2, 2]), (32, 10, 4, True, True, [0, 0, 0, 0, 1, 1, 1, 1, 2, 2]),
+                (33, 7, 3, True, False, [0, 0, 0, 1, 1, 1, -1])]
+S1R = np.array([0.3, 0.1, 0.06, 0.03], np.float32)
+S2R = np.array([0.08] * 4, np.float32)
+
+
+def noisy_scan_scene(seed, W):
     scans, poses = synth.make_scan_scene(seed, W=W, n_per_scan=2500)
     rng = np.random.default_rng(seed)
     noisy = poses.copy()
     for i in range(W):
         noisy[i, :9] = (noisy[i, :9].reshape(3, 3) @ synth.so3_exp(rng.normal(0, 0.004, (1, 3)))[0]).ravel(); noisy[i, 9:] += rng.normal(0, 0.01, 3)
-    s1r = np.array([0.3, 0.1, 0.06, 0.03], np.float32); s2r = np.array([0.08] * 4, np.float32)
-    sr.set_eigen_ratio_array(s1r)                                  # a fresh process: bavoxel.hpp:17
+    return scans, noisy
+
+
+def ref_lidar_ba(seed, W, win, use_rel, stage1, window_stage=True):
+    """The reference's runLidarBA on noisy_scan_scene(seed, W)."""
+    scans, noisy = noisy_scan_scene(seed, W)
+    sr.set_eigen_ratio_array(S1R)                                  # a fresh process: bavoxel.hpp:17
     S = sr.System()
     S.set_lidar(scans, noisy)
-    S.set_stages(True, win, 0.1, use_rel, stage1, 1.0, s1r, 0.5, s2r)
+    S.set_stages(window_stage, win, 0.1, use_rel, stage1, 1.0, S1R, 0.5, S2R)
     out = S.run_lidar_ba()
     S.close()
-    idx, _, _, final = lidar_chain(use_rel, scans, noisy, win, 0.1, (1.0, s1r), (0.5, s2r), stage1)
+    return dict(poses=out)
+
+
+@pytest.mark.parametrize("seed,W,win,use_rel,stage1,index", RAGGED_CASES)
+def test_lidar_half_live_ragged_windows_and_stage_switches(seed, W, win, use_rel, stage1, index):
+    """A last window shorter than the others, a last window of ONE frame (no voxel can see two poses: skipped, its frame keeps the odometry pose),
+    BALM_stage1/enable = false, both settings of use_window_ba_rel: the reference's runLidarBA against the oracle chain."""
+    scans, noisy = noisy_scan_scene(seed, W)
+    out = recorded(f"lidar_ba_{seed}")["poses"]
+    idx, _, _, final = lidar_chain(use_rel, scans, noisy, win, 0.1, (1.0, S1R), (0.5, S2R), stage1)
     assert idx.tolist() == index
     assert np.abs(out - final).max() <= 1e-9 and np.abs(out - noisy).max() > 1e-3
 
@@ -253,13 +283,24 @@ def test_ascending_order_is_a_different_but_documented_choice():
     assert len(tr) == 63 and mine <= {tuple(sorted(r)) for r in ref}                            # every ascending-order track is a reference track
 
 
-@needs_ref
-def test_libstdcxx_order_restatement_equals_the_real_container():
+def container_order_cases():
     rng = np.random.default_rng(0)
     for _ in range(2000):
         res = int(rng.integers(1, 60))
-        keys = rng.choice(90, size=int(rng.integers(1, min(res, 40) + 1)), replace=False).tolist()
-        assert sr.unordered_map_order(res, keys) == fo.libstdcxx_order(res, keys), (res, keys)
+        yield res, rng.choice(90, size=int(rng.integers(1, min(res, 40) + 1)), replace=False).tolist()
+
+
+def ref_container_order():
+    """The order std::unordered_map (reserve(res), then the keys inserted) visits its keys in, for every case."""
+    order, ptr = flat([np.array(sr.unordered_map_order(res, keys), np.int8) for res, keys in container_order_cases()])
+    return dict(order=order, ptr=ptr)
+
+
+def test_libstdcxx_order_restatement_equals_the_real_container():
+    R = recorded("container_order")
+    for k, (res, keys) in enumerate(container_order_cases()):
+        assert R["order"][R["ptr"][k]:R["ptr"][k + 1]].tolist() == fo.libstdcxx_order(res, keys), (res, keys)
+    assert k + 1 == len(R["ptr"]) - 1
 
 
 # ------------------------------------------------------------------------------------------------ P
@@ -288,7 +329,6 @@ def test_problem_handed_to_ceres():
         assert np.array_equal(G["P_obs_uv"][rows], uv)
 
 
-@needs_ref
 def test_points_and_planes_of_the_problem_against_the_oracle_chain_live():
     """Rebuilds the scene (2.9 MB of scans, not stored): usable tracks (:1432-1438), anchor clouds (:1471-1490), surf map under the eigen-ratio array
     in force (:1498-1506), recompute_local_planes (:1529-1566) out of the stage oracles vs what the reference recorded."""
@@ -333,23 +373,51 @@ def test_fixture_is_what_the_reference_pipeline_source_computes_bit_for_bit():
     assert exact or os.environ.get("LVBA_ALLOW_OTHER_HOST", "1") == "1"     # on the machine that wrote the file the regeneration is bit for bit
 
 
-# ------------------------------------------------------------------------------------------------ N4: the COLMAP database reader
 @needs_ref
+def test_live_fixtures_are_what_the_reference_source_computes():
+    """tests/golden/ref_live_balm.npz and ref_live_system.npz, which the *_live_* / differential / reader / loader / writer tests of this file
+    and of tests/test_ref_pin.py compare with, recomputed from the reference source by tests/golden/make_golden_ref_live.py."""
+    sys.path.insert(0, str(ROOT / "tests" / "golden"))
+    import make_golden_ref_live
+    for path, fresh in make_golden_ref_live.generate().items():
+        with np.load(path) as stored:
+            assert sorted(fresh) == sorted(stored.files), path.name
+            for k in stored.files:
+                a, b = np.asarray(fresh[k]), stored[k]
+                if a.dtype.kind in "iubU":
+                    assert np.array_equal(a, b), k                          # counts, keys, indices, flags, text: always
+                else:                                                       # another host CPU may round the last bits differently
+                    assert a.shape == b.shape and np.allclose(a, b, rtol=1e-9, atol=1e-11, equal_nan=True), k
+
+
+# ------------------------------------------------------------------------------------------------ N4: the COLMAP database reader
+def colmap_db_scene(root):
+    import visual_scene as vs
+    return vs.make(root, seed=5, W=6, n_per_scan=4000, n_landmarks=120)
+
+
+def ref_colmap_db_reader():
+    import visual_scene as vs
+    root = Path(tempfile.mkdtemp())
+    g = colmap_db_scene(root)
+    S = sr.System()
+    S.set_lidar(g["scans"][:1], g["poses"][:1], g["ts"][:1])
+    S.set_camera(g["width"], g["height"], g["intr"], vs.RCL.ravel(), vs.PCL, np.eye(3).ravel(), np.zeros(3), np.array(g["image_ts"]), g["image_poses"])
+    ok, kp_ptr, kp_uv, m = S.load_colmap_db(str(root) + "/", root / "Colmap" / "colmap.db")
+    S.close()
+    return dict(ok=ok, kp_ptr=kp_ptr, kp_uv=kp_uv, matches=m)
+
+
 def test_reference_reader_reads_the_database_the_dataset_writer_writes():
     """loadFromColmapDB (src/lvba_system.cpp:510-685, run from its own source against the system's SQLite) on the database
     oracle/dataset_writer.py wrote: database ids shuffled (so some pairs are stored with swapped columns, :655-660), one match with an
     out-of-range keypoint (dropped, :668-672).  It must hand back exactly the scene's keypoints and matches in the order
     BuildTracksAndFuse3D visits them — the same truth tests/test_visual_offline.py holds the product's own reader
     (global-lvba_b200/host/lvba_visual_offline.hpp) against."""
-    import visual_scene as vs
-    root = Path(tempfile.mkdtemp())
-    g = vs.make(root, seed=5, W=6, n_per_scan=4000, n_landmarks=120)
+    g = colmap_db_scene(Path(tempfile.mkdtemp()))
     assert sorted(g["db_ids"]) != g["db_ids"]
-    S = sr.System()
-    S.set_lidar(g["scans"][:1], g["poses"][:1], g["ts"][:1])
-    S.set_camera(g["width"], g["height"], g["intr"], vs.RCL.ravel(), vs.PCL, np.eye(3).ravel(), np.zeros(3), np.array(g["image_ts"]), g["image_poses"])
-    ok, kp_ptr, kp_uv, m = S.load_colmap_db(str(root) + "/", root / "Colmap" / "colmap.db")
-    S.close()
+    R = recorded("colmap_db_reader")
+    ok, kp_ptr, kp_uv, m = bool(R["ok"]), R["kp_ptr"], R["kp_uv"], R["matches"]
     assert ok
     assert np.array_equal(np.diff(kp_ptr), [len(k) for k in g["keypoints"]]) and np.array_equal(kp_uv, np.concatenate(g["keypoints"]))
     M = len(g["keypoints"])
@@ -360,7 +428,33 @@ def test_reference_reader_reads_the_database_the_dataset_writer_writes():
 
 
 # ------------------------------------------------------------------------------------------------ N4: the dataset loader
-@needs_ref
+def loader_dataset(root):
+    """The dataset the loader test reads, written under root; returns what was written."""
+    from oracle import dataset_writer as dw
+    scans, poses = synth.make_scan_scene(3, W=7, n_per_scan=900)
+    scans[4] = scans[4][:0]                                              # an empty scan file
+    ts = dw.write_lidar_dataset(root, scans, poses)                       # binary, ascii and LZF-compressed PCD files in turn
+    (root / "all_pcd_body" / "notes.txt").write_text("ignored")
+    image_ts = [t + 0.013 for t in ts]
+    image_poses = poses.copy(); image_poses[:, 9:] += np.random.default_rng(1).normal(0, 0.02, (7, 3))
+    dw.write_image_set(root, image_ts, image_poses, extra_between=1)
+    return scans, poses, ts, image_ts, image_poses
+
+
+def ref_dataset_loader():
+    """What DatasetIO's constructor read; its two paths with the dataset's directory taken off the front."""
+    root = Path(tempfile.mkdtemp())
+    loader_dataset(root)
+    S = sr.System({"data_config/data_path": str(root) + "/", "data_config/colmap_db_path": "Colmap/colmap.db", "data_config/image_sample_step": 2,
+                   "cam_model/cam_width": 160, "cam_model/cam_height": 128, "cam_model/scale": 0.5, "cam_model/cam_fx": 96.0, "cam_model/cam_fy": 96.3,
+                   "cam_model/cam_cx": 79.7, "cam_model/cam_cy": 64.2})
+    d = S.dataset()
+    S.close()
+    assert d["data_path"].startswith(str(root)) and d["db_path"].startswith(str(root))
+    xyz, scan_ptr = flat(d.pop("scans"))
+    return dict(d, scans_xyz=xyz, scan_ptr=scan_ptr, data_path=d["data_path"][len(str(root)):], db_path=d["db_path"][len(str(root)):])
+
+
 def test_reference_loader_reads_the_dataset_the_dataset_writer_writes():
     """DatasetIO's constructor (src/dataset_io.cpp, run from its own source; PCD files through the stand-in reader of oracle/ref_shim/pcl/io/pcd_io.h)
     on the directory oracle/dataset_writer.py lays out — the layout
@@ -369,20 +463,10 @@ def test_reference_loader_reads_the_dataset_the_dataset_writer_writes():
     image_sample_step-th file by timestamp and the same stride over the VALID pose lines (:118-121, :159), intrinsics scaled by cam_model/scale (:59-62),
     colmap_db_path appended to the data path (:65)."""
     from oracle import dataset_writer as dw
-    root = Path(tempfile.mkdtemp())
-    scans, poses = synth.make_scan_scene(3, W=7, n_per_scan=900)
-    scans[4] = scans[4][:0]                                              # an empty scan file
-    ts = dw.write_lidar_dataset(root, scans, poses)                       # binary, ascii and LZF-compressed PCD files in turn
-    (root / "all_pcd_body" / "notes.txt").write_text("ignored")
-    image_ts = [t + 0.013 for t in ts]
-    image_poses = poses.copy(); image_poses[:, 9:] += np.random.default_rng(1).normal(0, 0.02, (7, 3))
-    dw.write_image_set(root, image_ts, image_poses, extra_between=1)
-    S = sr.System({"data_config/data_path": str(root) + "/", "data_config/colmap_db_path": "Colmap/colmap.db", "data_config/image_sample_step": 2,
-                   "cam_model/cam_width": 160, "cam_model/cam_height": 128, "cam_model/scale": 0.5, "cam_model/cam_fx": 96.0, "cam_model/cam_fy": 96.3,
-                   "cam_model/cam_cx": 79.7, "cam_model/cam_cy": 64.2})
-    d = S.dataset()
-    S.close()
-    assert d["data_path"] == str(root) + "/" and d["db_path"] == str(root) + "/Colmap/colmap.db"
+    scans, poses, ts, image_ts, image_poses = loader_dataset(Path(tempfile.mkdtemp()))
+    d = recorded("dataset_loader")
+    d["scans"] = split(d["scans_xyz"], d["scan_ptr"])
+    assert str(d["data_path"]) == "/" and str(d["db_path"]) == "/Colmap/colmap.db"
     assert d["cam"][:6].tolist() == [80.0, 64.0, 48.0, 48.15, 39.85, 32.1] and d["cam"][10:].tolist() == [0.5, 2.0]
     assert np.array_equal(d["frame_ts"], np.array(ts))                   # from the names: the TUM file's own timestamps (0, 1, 2 ...) are ignored
     assert [len(s) for s in d["scans"]] == [len(s) for s in scans] and all(np.array_equal(a, b) for a, b in zip(d["scans"], scans))
@@ -394,7 +478,14 @@ def test_reference_loader_reads_the_dataset_the_dataset_writer_writes():
 
 
 # ------------------------------------------------------------------------------------------------ B5: the per-track helpers on their own
-@needs_ref
+def ref_track_helpers():
+    import test_track_emu as tt
+    p, cams, op, oc, uv, intr = tt._problem()
+    Xr, mr, cr, okr = sr.track_helpers(op, oc, uv, cams, intr)
+    _, m2, c2, ok2 = sr.track_helpers(op, oc, uv, cams, intr, Xw=np.ascontiguousarray(p["X_gt"] + 0.01), min_count=5)
+    return dict(X=Xr, mean=mr, count=cr, ok=okr, mean_at_X=m2, count_at_X=c2, ok_at_X=ok2)
+
+
 def test_dlt_and_mean_reprojection_equal_reference_source_live():
     """TriangulateTrackDLT (src/lvba_system.cpp:52-111) and ComputeMeanReproj (:8-50), called directly (they are file-scope functions of the
     included source), vs oracle/track_oracle.py and the device functors through the host policy (tests/emu/track_emu.cpp) on 400 tracks.
@@ -406,7 +497,8 @@ def test_dlt_and_mean_reprojection_equal_reference_source_live():
     from oracle import track_oracle as tro
     p, cams, op, oc, uv, intr = tt._problem()
     T = len(op) - 1
-    Xr, mr, cr, okr = sr.track_helpers(op, oc, uv, cams, intr)
+    R = recorded("track_helpers")
+    Xr, mr, cr, okr = R["X"], R["mean"], R["count"], R["ok"]
     so = Path(tempfile.mkdtemp()) / "libtrack_emu.so"
     r = subprocess.run(["g++", "-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-shared", str(ROOT / "tests" / "emu" / "track_emu.cpp"), "-o", str(so)],
                        capture_output=True, text=True)
@@ -424,7 +516,7 @@ def test_dlt_and_mean_reprojection_equal_reference_source_live():
         o_ok, X, m, c = tro.triangulate_dlt(cams[oc[sel]], uv[sel], intr)
         assert o_ok and c == cr[t] and np.abs(X - Xr[t]).max() <= 1e-7 * max(1.0, np.abs(X).max()) and abs(m - mr[t]) <= 1e-7   # LAPACK eigh vs Jacobi on short baselines: the smallest eigenvector of A^T A is conditioned like 1e7
     X = np.ascontiguousarray(p["X_gt"] + 0.01)
-    _, m2, c2, ok2 = sr.track_helpers(op, oc, uv, cams, intr, Xw=X, min_count=5)
+    m2, c2, ok2 = R["mean_at_X"], R["count_at_X"], R["ok_at_X"]
     assert ok2.any() and not ok2.all()
     for t in range(0, T, 5):
         sel = list(range(op[t], op[t + 1]))
@@ -452,9 +544,21 @@ def _depth_images_for(s, width=640, height=512):
     return img
 
 
-@needs_ref
-@pytest.mark.parametrize("seed,kw", [(0, {}), (1, dict(wrong=0.15)), (2, dict(no_depth=0.6)), (3, dict(bad_depth=0.3, px_noise=1.2)),
-                                     (4, dict(n_images=30, n_points=300)), (7, dict(n_images=45, n_points=200, wrong=0.1)), (8, dict(n_images=20, n_points=150, wrong=0.3))])
+FUSION_CASES = [(0, {}), (1, dict(wrong=0.15)), (2, dict(no_depth=0.6)), (3, dict(bad_depth=0.3, px_noise=1.2)),
+                (4, dict(n_images=30, n_points=300)), (7, dict(n_images=45, n_points=200, wrong=0.1)), (8, dict(n_images=20, n_points=150, wrong=0.3))]
+
+
+def ref_build_tracks(seed, kw):
+    import fuse_scene
+    s = fuse_scene.make(seed=seed, **kw)
+    S = sr.System()
+    S.set_fusion_inputs(s["cams"], _depth_images_for(s), s["intr"], s["kp_ptr"], s["kp_uv"], s["matches"])
+    T = S.build_tracks()
+    S.close()
+    return T
+
+
+@pytest.mark.parametrize("seed,kw", FUSION_CASES)
 def test_track_fusion_differential_reference_source_vs_oracle_and_device_pass(seed, kw, tmp_path_factory):
     """BuildTracksAndFuse3D from the reference's own source on the scenes of tests/test_fuse_emu.py (wrong matches that merge components, missing and
     wrong depth, up to 45 images: more keys than buckets in the reference's maps, failed components retried from other seeds) against
@@ -466,10 +570,7 @@ def test_track_fusion_differential_reference_source_vs_oracle_and_device_pass(se
     s = fuse_scene.make(seed=seed, **kw)
     depth = _depth_images_for(s)
     Xw, valid = dep.backproject(list(depth), s["cams"], s["intr"], s["kp_ptr"], s["kp_uv"])
-    S = sr.System()
-    S.set_fusion_inputs(s["cams"], depth, s["intr"], s["kp_ptr"], s["kp_uv"], s["matches"])
-    T = S.build_tracks()
-    S.close()
+    T = recorded(f"build_tracks_{seed}")
     tr = fo.fuse(s["kp_ptr"], s["kp_uv"], s["matches"], s["cams"], s["intr"], Xw, valid, map_order=fo.libstdcxx_order)
     assert len(tr) == len(T["Xw"]) > 0
     for k, t in enumerate(tr):
@@ -492,14 +593,18 @@ def test_track_fusion_differential_reference_source_vs_oracle_and_device_pass(se
 
 
 # ------------------------------------------------------------------------------------------------ D, differential: more scenes, live
-@needs_ref
-@pytest.mark.parametrize("seed,F,M,size", [(11, 5, 3, (64, 48)), (12, 9, 6, (120, 90)), (13, 4, 5, (200, 160))])
-def test_depth_rendering_differential_reference_source_vs_oracle(seed, F, M, size):
-    """buildGridMapFromOptimized + generateDepthWithVoxel from the reference's own source on further scenes (image timestamps outside the scan range
-    included: some images see no frame) — images equal to the oracle's bit for bit."""
+DEPTH_CASES = [(11, 5, 3, (64, 48)), (12, 9, 6, (120, 90)), (13, 4, 5, (200, 160))]
+
+
+def depth_scene_for(seed, F, M, size):
     sc = synth.make_depth_scene(seed, F=F, n_per_scan=1800, M=M, width=size[0], height=size[1])
     img_ts = np.round(sc["image_ts"], 6)
     img_ts[0] = sc["frame_ts"][0] - 3.0                                   # nothing within +-0.5 s: an empty image
+    return sc, img_ts
+
+
+def ref_depth(seed, F, M, size):
+    sc, img_ts = depth_scene_for(seed, F, M, size)
     body = np.zeros((M, 12))
     for k in range(M):                                                    # body poses whose cameras are sc["cams"]: Rcw = Rci Rwi^T with Rci = I, tci = 0
         Rcw = sc["cams"][k, :9].reshape(3, 3); tcw = sc["cams"][k, 9:]
@@ -511,27 +616,64 @@ def test_depth_rendering_differential_reference_source_vs_oracle(seed, F, M, siz
     S.build_grid(); S.update_camera_poses()
     d, _, c1 = S.generate_depth()
     S.close()
+    return dict(depth=d, cams=c1)
+
+
+@pytest.mark.parametrize("seed,F,M,size", DEPTH_CASES)
+def test_depth_rendering_differential_reference_source_vs_oracle(seed, F, M, size):
+    """buildGridMapFromOptimized + generateDepthWithVoxel from the reference's own source on further scenes (image timestamps outside the scan range
+    included: some images see no frame) — images equal to the oracle's bit for bit."""
+    sc, img_ts = depth_scene_for(seed, F, M, size)
+    R = recorded(f"depth_{seed}")
+    d, c1 = R["depth"], R["cams"]
     assert np.abs(c1 - sc["cams"]).max() <= 1e-12
     img = dep.render(sc["scans"], sc["poses"], sc["frame_ts"], c1, img_ts, sc["intr"], size[0], size[1])
     assert np.array_equal(img, d) and not d[0].any() and (d[1:] > 0).sum() > 500
 
 
 # ------------------------------------------------------------------------------------------------ N4: the COLMAP text model
-@needs_ref
-def test_colmap_export_equals_the_reference_writer(pkg, tmp_path):
-    """VisualizeOptComparison (src/lvba_system.cpp:1932-2143), run from its own source on a dataset its own loader read (every image file = one grey value:
-    there is no decoder on either side), against `lvba_offline --check --visual --points3d lidar` (host code of global-lvba_b200/host/lvba_visual_offline.hpp,
-    no GPU): images.txt line for line, points3D.txt row for row as a set (the reference lists the thinned points in unordered_map order)."""
-    import subprocess
+def colmap_export_dataset(data):
     import visual_scene as vs
     from oracle import dataset_writer as dw
-    data = tmp_path / "data"
     g = vs.make(data, seed=4, W=6, n_per_scan=6000, n_landmarks=60)
     # one more image 5 s after the last scan: no LiDAR within +-0.5 s -> the reference lists it neither in images.txt nor in the points (:1994-1997)
     image_ts = list(g["image_ts"]) + [g["image_ts"][-1] + 5.0]
     image_poses = np.vstack([g["image_poses"], g["image_poses"][-1:]])
     dw.write_image_set(data, image_ts, image_poses, extra_between=1)
     dw.write_colmap_db(data / "Colmap" / "colmap.db", image_ts, g["keypoints"] + [np.zeros((0, 2), np.float32)], {k: np.array(v) for k, v in g["pair"].items() if k != (0, 1)})
+
+
+def points3d_rows(text):
+    return sorted(" ".join(ln.split()[1:]) for ln in text.splitlines())
+
+
+def ref_colmap_export():
+    """The reference's images.txt and the rows of its points3D.txt (point ids dropped, sorted) on colmap_export_dataset."""
+    import visual_scene as vs
+    data = Path(tempfile.mkdtemp()) / "data"
+    colmap_export_dataset(data)
+    F = vs.INTR_FULL
+    S = sr.System({"data_config/data_path": str(data) + "/", "data_config/colmap_db_path": "Colmap/colmap.db", "data_config/image_sample_step": 2,
+                   "cam_model/cam_width": vs.WIDTH_FULL, "cam_model/cam_height": vs.HEIGHT_FULL, "cam_model/scale": vs.SCALE, "cam_model/cam_fx": F[0],
+                   "cam_model/cam_fy": F[1], "cam_model/cam_cx": F[2], "cam_model/cam_cy": F[3], "cam_model/cam_d0": F[4], "cam_model/cam_d1": F[5],
+                   "cam_model/cam_d2": F[6], "cam_model/cam_d3": F[7], "extrin_calib/Rcl": vs.RCL.ravel(), "extrin_calib/Pcl": vs.PCL,
+                   "extrin_calib/extrinsic_R": np.eye(3).ravel(), "extrin_calib/extrinsic_T": np.zeros(3)})
+    d = S.init_from_dataset()
+    S.build_grid(); S.update_camera_poses(); S.generate_depth()
+    S.colmap_export(str(data) + "/")
+    S.close()
+    ref_dir = data / "Colmap" / "sparse"
+    return dict(n_frames=len(d["frame_ts"]), n_images=len(d["image_ts"]), images_txt=(ref_dir / "images.txt").read_text(),
+                points3d_rows="\n".join(points3d_rows((ref_dir / "points3D.txt").read_text())))
+
+
+def test_colmap_export_equals_the_reference_writer(pkg, tmp_path):
+    """VisualizeOptComparison (src/lvba_system.cpp:1932-2143), run from its own source on a dataset its own loader read (every image file = one grey value:
+    there is no decoder on either side), against `lvba_offline --check --visual --points3d lidar` (host code of global-lvba_b200/host/lvba_visual_offline.hpp,
+    no GPU): images.txt line for line, points3D.txt row for row as a set (the reference lists the thinned points in unordered_map order)."""
+    import subprocess
+    data = tmp_path / "data"
+    colmap_export_dataset(data)
     exe = tmp_path / "lvba_offline"
     cmd = ["g++", "-std=c++17", "-O2", "-I", str(ROOT / "include"), str(ROOT / "tools" / "lvba_offline.cpp"), "-o", str(exe),
            str(pkg.LIB_PATH), f"-Wl,-rpath,{pkg.LIB_PATH.parent}", "-L/usr/local/cuda/lib64", "-lcudart", "-ldl"]
@@ -541,49 +683,35 @@ def test_colmap_export_equals_the_reference_writer(pkg, tmp_path):
     r = subprocess.run([str(exe), "--data", str(data), "--config", str(data / "config.yaml"), "--check", "--visual", "--points3d", "lidar", "--sparse-dir", str(mine)],
                        capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout + r.stderr
-    F = vs.INTR_FULL
-    S = sr.System({"data_config/data_path": str(data) + "/", "data_config/colmap_db_path": "Colmap/colmap.db", "data_config/image_sample_step": 2,
-                   "cam_model/cam_width": vs.WIDTH_FULL, "cam_model/cam_height": vs.HEIGHT_FULL, "cam_model/scale": vs.SCALE, "cam_model/cam_fx": F[0],
-                   "cam_model/cam_fy": F[1], "cam_model/cam_cx": F[2], "cam_model/cam_cy": F[3], "cam_model/cam_d0": F[4], "cam_model/cam_d1": F[5],
-                   "cam_model/cam_d2": F[6], "cam_model/cam_d3": F[7], "extrin_calib/Rcl": vs.RCL.ravel(), "extrin_calib/Pcl": vs.PCL,
-                   "extrin_calib/extrinsic_R": np.eye(3).ravel(), "extrin_calib/extrinsic_T": np.zeros(3)})
-    d = S.init_from_dataset()
-    assert len(d["frame_ts"]) == 6 and len(d["image_ts"]) == 7
-    S.build_grid(); S.update_camera_poses(); S.generate_depth()
-    S.colmap_export(str(data) + "/")
-    S.close()
-    ref_dir = data / "Colmap" / "sparse"
-    assert (mine / "images.txt").read_text() == (ref_dir / "images.txt").read_text()
-    assert len((ref_dir / "images.txt").read_text().splitlines()) == 12          # six of the seven images: the late one is left out on both sides
-    rows = lambda f: sorted(" ".join(ln.split()[1:]) for ln in f.read_text().splitlines())  # noqa: E731
-    a, b = rows(mine / "points3D.txt"), rows(ref_dir / "points3D.txt")
+    R = recorded("colmap_export")
+    assert int(R["n_frames"]) == 6 and int(R["n_images"]) == 7
+    ref_images = str(R["images_txt"])
+    assert (mine / "images.txt").read_text() == ref_images
+    assert len(ref_images.splitlines()) == 12                                     # six of the seven images: the late one is left out on both sides
+    a, b = points3d_rows((mine / "points3D.txt").read_text()), str(R["points3d_rows"]).split("\n")
     assert len(a) == len(b) > 2000 and a == b
     assert all(ln.endswith("128 128 128 0") for ln in a[:50])
 
 
-@needs_ref
 def test_lidar_half_live_without_the_window_stage():
     """window_ba/enable = false (:217-225): the global stages run on the frames themselves — the path `lvba_offline` takes without --window."""
-    scans, poses = synth.make_scan_scene(41, W=6, n_per_scan=2500)
-    rng = np.random.default_rng(41)
-    noisy = poses.copy()
-    for i in range(6):
-        noisy[i, :9] = (noisy[i, :9].reshape(3, 3) @ synth.so3_exp(rng.normal(0, 0.004, (1, 3)))[0]).ravel(); noisy[i, 9:] += rng.normal(0, 0.01, 3)
-    s1r = np.array([0.3, 0.1, 0.06, 0.03], np.float32); s2r = np.array([0.08] * 4, np.float32)
-    sr.set_eigen_ratio_array(s1r)
-    S = sr.System()
-    S.set_lidar(scans, noisy)
-    S.set_stages(False, 10, 0.1, False, True, 1.0, s1r, 0.5, s2r)
-    out = S.run_lidar_ba()
-    S.close()
+    scans, noisy = noisy_scan_scene(41, 6)
+    out = recorded("lidar_ba_41")["poses"]
     x = noisy
-    for vs_, er in ((1.0, s1r), (0.5, s2r)):
+    for vs_, er in ((1.0, S1R), (0.5, S2R)):
         vp, pi, cl, _ = vox.voxelize(scans, x, vs_, er)
         x, _ = lo.damping_iter(vp, pi, cl, x)
     assert np.abs(out - x).max() <= 1e-9 and np.abs(out - noisy).max() > 1e-3
 
 
-@needs_ref
+def bucket_count_ns():
+    return list(range(0, 300)) + [p + d for p in fo._PRIMES if p < 3_000_000 for d in (-1, 0, 1)]
+
+
+def ref_bucket_counts():
+    return dict(n=np.array(bucket_count_ns(), np.int64), bucket_count=np.array([sr.bucket_count_after_reserve(n) for n in bucket_count_ns()], np.int64))
+
+
 def test_bucket_count_table_equals_the_real_container(tmp_path_factory):
     """stl_bucket_count (csrc/fuse_pipeline.h) and the table of oracle/fuse_oracle.py against std::unordered_map::reserve(n) / bucket_count() of the
     library the reference is compiled with: every n up to 300, then every table entry below 3e6 and its two neighbours."""
@@ -594,9 +722,10 @@ def test_bucket_count_table_equals_the_real_container(tmp_path_factory):
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     lib = ctypes.CDLL(str(so)); lib.emu_stl_bucket_count.restype = ctypes.c_uint
-    ns = list(range(0, 300)) + [p + d for p in fo._PRIMES if p < 3_000_000 for d in (-1, 0, 1)]
-    for n in ns:
-        real = sr.bucket_count_after_reserve(n)
+    R = recorded("bucket_counts")
+    ns = bucket_count_ns()
+    assert R["n"].tolist() == ns
+    for n, real in zip(ns, R["bucket_count"].tolist()):
         assert lib.emu_stl_bucket_count(ctypes.c_uint(n)) == real, n
         if n >= 14:
             assert next(p for p in fo._PRIMES if p >= n) == real, n
